@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric: megapixels/s of fused BilateralSliceApply @4K.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is ONE pass of the hot path over one batch of synthetic input: one launch of the fused
@@ -14,6 +14,10 @@ per GPU); timing is CUDA events on the launch stream, max over ranks.
 Rank 0 prints ONE JSON line (keys: see the task contract).  `--impl reference` times the
 reference's own CPU loops (oracle/_ref: hdrnet/ops/bilateral_slice_apply.cc compiled
 unmodified; falls back to the C restatement) on the host cores.
+
+`--dump-outputs DIR` writes, after the timed steps, a fixed seeded sample of what the last timed
+step returned (see dump_outputs): the inputs are seeded too, so two builds can be compared value
+for value.  The bench writes nothing into the source tree, which may be read-only.
 """
 from __future__ import annotations
 
@@ -29,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ written into the tree by the imports below
 
 METRIC = "megapixels/s BilateralSliceApply @4K"
 UNIT = "MP/s"
@@ -136,13 +141,7 @@ def cpu_checker():
     if os.environ.get("OMP_NUM_THREADS") in (None, "1"):
         os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)
     import oracle
-    if not oracle.have_ref() or not os.path.exists(os.path.join(ROOT, "oracle", "_build",
-                                                                "libhdrnet_oracle.so")):
-        try:
-            oracle.build()
-        except Exception:
-            pass
-    return oracle.best()
+    return oracle.best()       # the checkers __graft_entry__.build() compiled; nothing is built here
 
 
 def cpu_inputs(frames: int, rows: int, seed: int = 1234):
@@ -359,6 +358,20 @@ def extra_records(torch, dist, lib, _lib, dev, stream, world, rank, peak, args):
 # ------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------
+DUMP_PIXELS = 1 << 20   # 12 MB of float32 RGB out of the 796 MB output of one step
+
+
+def dump_outputs(torch, out, directory, name, pixels):
+    """Writes `pixels` output pixels of the last timed step to directory/name.npy, float32 [pixels, N_OUT].
+    The pixels are a seeded sample (numpy default_rng(0), sorted flat pixel indices into out[B,H,W]),
+    the same on every run, so two builds' files compare element for element."""
+    flat = out.view(-1, out.shape[-1])
+    idx = np.sort(np.random.default_rng(0).choice(flat.shape[0], size=min(pixels, flat.shape[0]), replace=False))
+    sample = flat.index_select(0, torch.from_numpy(idx).to(out.device)).cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name + ".npy"), sample.astype(np.float32))
+
+
 def run_b200_arm(args):
     import torch
     import torch.distributed as dist
@@ -436,6 +449,9 @@ def run_b200_arm(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     elapsed_max_ms = float(t.item())
     own_launch_ms = elapsed_ms / args.steps
+    if args.dump_outputs:       # before any later leg runs the step again
+        dump_outputs(torch, out, args.dump_outputs, "out" if world == 1 else f"out_rank{rank}",
+                     DUMP_PIXELS // world)
 
     # ---- end to end: public API, pinned HOST buffers, H2D + kernel + D2H inside the timing --
     e2e_steps = max(1, min(args.steps, args.e2e_steps))
@@ -574,7 +590,14 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra records (configs 2, 4, 5, model path)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of the last step's output to DIR/out.npy "
+                         "(DIR/out_rank<r>.npy per rank when several GPUs run)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's output; --impl reference has none")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_b200_arm(args)

@@ -1,6 +1,7 @@
 """Generate the golden fixtures in tests/golden/ from the REFERENCE itself.
 
-Run in the build container (needs /root/reference):   python tests/golden/make_golden.py
+Needs the reference's sources (oracle/jax_shim.py imports its JAX file; oracle/_ref is built from its
+.cc files by oracle/Makefile):   python tests/golden/make_golden.py [jax | vjp | ref]
 
 Outputs are produced by the reference's own jax/bilateral_slice.py (:299-380), imported
 unmodified under the numpy stand-in for jax (oracle/jax_shim.py), and -- for slice-apply --
@@ -13,11 +14,20 @@ reference's tests:
                      from 640x480x4 to 2x96x128 to keep the fixture small)
   interpolate_kat    hdrnet/test/ops_test.py:61-86 (grid value = depth index)
   edge_cases         guide exactly 0 / 1 / out of [0,1], 1-pixel-wide image, gd = 1
+  signed_random      signed grid and input (tests/util.py rand_case(11, ...)) on a non-square grid
   vjp_*              the reference's own VJPs of the slice (jax/bilateral_slice.py:26-108, :257-295) at
                      the extents of its gradient tests (hdrnet_ops_test.py:91-100, :185-195) and on a
-                     grid coarser / finer than the image; `python make_golden.py vjp` writes only these
-Each .npz stores inputs, outputs and the reference's cell indices.
+                     grid coarser / finer than the image, and vjp_cell_centre: a guide on an exact
+                     depth-cell centre, where the JAX helpers and the C++ op differ
+  compiled_ref_sha256.json
+                     the reference's own C++ loops (oracle/_ref): forward at three extents and all five
+                     VJPs at hdrnet_ops_test.py:185-195's, on tests/util.py rand_case inputs.  The C
+                     restatement must match them bit for bit, so only the SHA-256 of each output's
+                     float32 bytes is stored
+Each forward .npz stores inputs, outputs and the reference's cell indices.
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -25,6 +35,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.normpath(os.path.join(HERE, "..", "..")))
+sys.path.insert(0, os.path.normpath(os.path.join(HERE, "..")))
 
 from oracle import jax_shim  # noqa: E402
 
@@ -89,9 +100,13 @@ def main():
 
     # Wide enough for the TMA row kernel (W % 4 == 0, W >= 128), ragged last segment.
     grid = rng.rand(2, 4, 6, 8, 12).astype(np.float32)
-    guide = rng.rand(2, 6, 1100).astype(np.float32)
-    inp = rng.rand(2, 6, 1100, 3).astype(np.float32)
+    guide = rng.rand(2, 5, 1100).astype(np.float32)
+    inp = rng.rand(2, 5, 1100, 3).astype(np.float32)
     save("wide_rows", **case(grid, guide, inp))
+
+    # Signed grid and input on a small non-square grid (tests/util.py draws them this way).
+    from util import rand_case
+    save("signed_random", **case(*rand_case(11, 2, 40, 36, 8, 6, 5, signed=True)))
 
 
 def main_vjp():
@@ -109,8 +124,59 @@ def main_vjp():
         gv, uv = jax_shim.bilateral_slice_vjp(grid, guide, ct)
         save(f"vjp_{k}", grid=grid, guide=guide, codomain_tangent=ct, grid_vjp=gv, guide_vjp=uv)
 
+    # One pixel's guide on the centre of depth cell 1 (guide * gd - 0.5 == 1 exactly in float32), zero grid:
+    # the inputs of tests/test_oracle.py's exact-cell-centre test.
+    gh, gw, gd, gc, h, w = 3, 2, 4, 1, 6, 5
+    rng = np.random.RandomState(11)
+    guide = rng.rand(1, h, w).astype(np.float32)
+    guide[0, 2, 3] = 1.5 / gd
+    ct = rng.randn(1, h, w, gc).astype(np.float32)
+    grid = np.zeros((1, gh, gw, gd, gc), np.float32)
+    gv, uv = jax_shim.bilateral_slice_vjp(grid, guide, ct)
+    save("vjp_cell_centre", grid=grid, guide=guide, codomain_tangent=ct, grid_vjp=gv, guide_vjp=uv)
+
+
+# tests/test_oracle.py test_port_is_bit_exact_with_compiled_reference's extents (B, H, W, gh, gw, gd)
+COMPILED_REF_SHAPES = [(3, 30, 25, 16, 12, 8), (2, 64, 48, 3, 5, 4), (1, 8, 5, 6, 3, 7)]
+
+
+def sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(a, np.float32).tobytes()).hexdigest()
+
+
+def main_compiled_ref():
+    import oracle
+    from util import rand_case
+    ref = oracle.ref()
+    digests = {}
+    for shape in COMPILED_REF_SHAPES:
+        grid, guide, inp = rand_case(99, *shape, signed=True)
+        digests["x".join(map(str, shape))] = {
+            "slice": sha256(ref.bilateral_slice(grid, guide)),
+            "apply_offset": sha256(ref.bilateral_slice_apply(grid, guide, inp, True)),
+            "apply_nooffset": sha256(ref.bilateral_slice_apply(grid, guide, inp, False))}
+    # the VJPs, as tests/test_oracle.py test_port_vjps_bit_exact_with_compiled_reference draws its inputs
+    B, H, W, gh, gw, gd, n_in, n_out = 3, 8, 5, 6, 3, 7, 3, 4
+    grid, guide, inp = rand_case(5, B, H, W, gh, gw, gd, n_in, n_out, True)
+    rng = np.random.RandomState(6)
+    ct = rng.rand(B, H, W, n_out).astype(np.float32)
+    vjp = dict(zip(("apply_grid", "apply_guide", "apply_input"),
+                   map(sha256, ref.bilateral_slice_apply_grad(grid, guide, inp, ct, True))))
+    ct = rng.rand(B, H, W, grid.shape[-1]).astype(np.float32)
+    vjp.update(zip(("slice_grid", "slice_guide"), map(sha256, ref.bilateral_slice_grad(grid, guide, ct))))
+    digests["vjp"] = vjp
+    path = os.path.join(HERE, "compiled_ref_sha256.json")
+    with open(path, "w") as f:
+        json.dump(digests, f, indent=1, sort_keys=True)
+        f.write("\n")
+    print(f"compiled_ref_sha256.json: {len(digests)} cases")
+
 
 if __name__ == "__main__":
-    if sys.argv[1:] != ["vjp"]:
+    what = sys.argv[1:] or ["jax", "vjp", "ref"]
+    if "jax" in what:
         main()
-    main_vjp()
+    if "vjp" in what:
+        main_vjp()
+    if "ref" in what:
+        main_compiled_ref()

@@ -45,7 +45,7 @@ def checker():
 # ---- golden fixtures from the reference's jax/bilateral_slice.py ---------------------------
 @pytest.mark.parametrize("name", ["ops_test_extents", "jax_tf2_extents", "interpolate_kat_0",
                                   "interpolate_kat_1", "interpolate_kat_2", "edge_guides",
-                                  "edge_gd1", "wide_rows"])
+                                  "edge_gd1", "wide_rows", "signed_random"])
 def test_matches_reference_jax_golden(name):
     g = load_golden(name)
     assert_parity(run_slice(g["grid"], g["guide"]), g["slice"], what=f"{name}: slice")
